@@ -21,6 +21,11 @@ A "step" is one pass of the hot path over one batch of synthetic stripes:
 `cpu_baseline` = the oracle's multi-threaded SIMD port (AVX2 nibble tables / GFNI as klauspost would
            select, + PCLMUL CRC32) on this box's host cores, bounded sample.
 
+`--dump-outputs DIR` = what the last timed step handed back, for comparing two builds output for output: the parity
+           shards (encode) or the regenerated shards (reconstruct) of the checked stripes and, with CRC, the CRCs of
+           every shard of the batch, as DIR/<name>.npy in float32 / float64 (rank 0; 45 MB or less).  The inputs are
+           seeded, so the same arguments give the same inputs on every run.
+
 python bench.py --gpus N --steps K --warmup W          (N>1: launched by torch.distributed.run)
 python bench.py --impl reference ...                   (the reference's CPU path = oracle port; rank 0 only)
 """
@@ -320,6 +325,7 @@ def main():
     ap.add_argument("--no-check", action="store_true")
     ap.add_argument("--force", type=int, default=0, help="cubeec_debug_force_kernel value (A/B aid, see include/cubeec.h)")
     ap.add_argument("--single-threads", default="64,256,1000", help="caller threads of the e2e_single_call record")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -436,6 +442,19 @@ def main():
                     raise SystemExit(f"bench check FAILED: reconstructed shard {i} of stripe {s} differs from the original")
         return len(sample_ids)
 
+    def last_step_outputs():
+        """What a caller of the timed path receives, for the checked stripes (bytes as float32, CRCs as float64: exact)."""
+        out = {"stripe_ids": np.asarray(sample_ids, dtype=np.float64)}
+        if args.workload == "reconstruct":
+            lost = [np.nonzero(present3[s] == 0)[0] for s in sample_ids]
+            out["erased_shards"] = np.asarray(lost, dtype=np.float64)
+            out["reconstructed"] = np.stack([host_stripe(s)[i] for s, i in zip(sample_ids, lost)]).astype(np.float32)
+        else:
+            out["parity"] = np.stack([host_stripe(s)[K:] for s in sample_ids]).astype(np.float32)
+            if args.crc:
+                out["crc32"] = dcrc.cpu().numpy().view(np.uint32).reshape(ns, n).astype(np.float64)
+        return out
+
     # ---- headline -------------------------------------------------------------------------------------------
     peak, peak_src = measured_peak()
     enc(True)
@@ -476,6 +495,10 @@ def main():
     checked = 0
     if not args.no_check:
         checked = check_reconstruct(originals, present3) if args.workload == "reconstruct" else check_encode(bool(args.crc))
+    if args.dump_outputs and rank == 0:   # before the extra records below run other kernels over the same batch
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in last_step_outputs().items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     def record(ms_, alg_bytes, kernel):
         ach = alg_bytes / (ms_ * 1e-3) / 1e9
@@ -487,7 +510,7 @@ def main():
     extra = None
     if world == 1 and not args.no_extra:
         extra = {}
-        st, wu = max(3, min(args.steps, 5)), 3
+        st, wu = args.steps, 3
         if args.workload == "reconstruct":
             rec(present3)   # leave the batch consistent
         ms_ = timed(lambda: enc(False), st, wu)
@@ -531,7 +554,7 @@ def main():
             crc_h, _ = eng.encode_contig(hnp, S, ns_e, n * S, crc=bool(args.crc))
         barrier()
         t0 = time.perf_counter()
-        reps = max(2, min(args.steps, 5))
+        reps = args.steps
         for _ in range(reps):
             eng.encode_contig(hnp, S, ns_e, n * S, crc=bool(args.crc))
         torch.cuda.synchronize(dev)
